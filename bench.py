@@ -572,6 +572,19 @@ def pin_to_gpu_numa_node(local):
         return None
 
 
+DUMP_PIXELS = 1 << 20   # 16 MiB as float32 BGRA
+
+
+def dump_framebuffer(out_dir, fb):
+    """The framebuffer a caller of the timed path reads back, as float32 BGRA values 0..255 of DUMP_PIXELS
+    pixels drawn with a fixed seed (row-major order), so that two builds can be compared output for output."""
+    import numpy as np
+    px = fb.reshape(-1, 4)
+    idx = np.sort(np.random.RandomState(0).choice(px.shape[0], DUMP_PIXELS, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "framebuffer.npy"), px[idx].astype(np.float32))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -586,7 +599,12 @@ def main():
     ap.add_argument("--sweep-only", action="store_true", help="only the layer-depth sweep (for an ncu pass over its kernels)")
     ap.add_argument("--workload", default="config_b",
                     help="config_b (the contract's bench line) or one of the other §8 rows: see other_workloads(), update_path")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="config_b: write what the last timed step drew to DIR/framebuffer.npy (float32 BGRA of a fixed "
+                         "seeded sample of 2^20 pixels) for output-for-output comparison of two builds")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "wrcu" or args.workload != "config_b" or args.sweep_only):
+        ap.error("--dump-outputs writes the config_b frame of --impl wrcu")
     args.warmup = max(args.warmup, 3) if args.impl == "wrcu" else args.warmup
 
     if args.impl == "reference":
@@ -675,6 +693,8 @@ def main():
         kernel_ms.append(dev.timer_end())
     barrier()
     st = dev.stats()
+    if rank == 0 and args.dump_outputs:
+        dump_framebuffer(args.dump_outputs, dev.read_pixels(tgt, 0, 0, W, H, 4))
     if rank == 0 and not sampler.lines:
         # a short timed region can end before nvidia-smi's first 100 ms sample: keep the same load
         # running (untimed) until one arrives, so the clocks line still describes the GPU under this work

@@ -27,9 +27,12 @@ def build():
         return LIB
     os.makedirs(os.path.dirname(LIB), exist_ok=True)
     renames = [f"-D{s}={s.replace('wrcu_', 'wremu_', 1)}" for s in abi.SYMBOLS]
+    # parallel test workers may build at once: each links its own file and renames it into place
+    tmp = f"{LIB}.{os.getpid()}"
     cmd = ["g++", "-x", "c++", "-std=c++17", "-O1", "-fPIC", "-shared", "-ffp-contract=off", "-fno-math-errno",
-           "-DWRCU_HOSTEMU", "-w"] + renames + ["-o", LIB, os.path.join(CSRC, "wrcu_api.cu"), "-lm"]
+           "-DWRCU_HOSTEMU", "-w"] + renames + ["-o", tmp, os.path.join(CSRC, "wrcu_api.cu"), "-lm"]
     subprocess.run(cmd, check=True)
+    os.replace(tmp, LIB)
     return LIB
 
 

@@ -8,7 +8,7 @@ from webrender_b200 import abi
 from workloads import scenes
 from webrender_b200.device import CudaDevice
 
-from common import assert_same, render
+from common import assert_same, reference, render  # noqa: F401 (reference: fixture)
 
 pytestmark = pytest.mark.gpu
 
@@ -538,20 +538,20 @@ def test_binned_batch_two_list_passes():
 
 
 # ---- perspective quads / plane-split polygons: against the reference build itself -------------------------
-# (oracle/_ref travels with the repo; the plain-C port does not restate draw_perspective)
+# (the plain-C port does not restate draw_perspective: the expected bytes are the host emulation's, which the
+# `reference` fixture holds to the digest of the reference build's output)
 PERSP_CAMERAS = [(800.0, 35.0, 0.0), (800.0, -20.0, 15.0), (220.0, 60.0, -30.0), (220.0, 80.0, 40.0), (150.0, -70.0, 55.0)]
 
 
-def _swgl():
-    from oracle.backends import SwglDevice, have_swgl
-    if not have_swgl():
-        pytest.skip("oracle/_ref (the reference build) not present")
-    return SwglDevice
+def _reference_pixels(reference, f, names):
+    from emu import EmuDevice
+    from oracle.backends import SwglDevice
+    return reference(render(EmuDevice, f, names), lambda: render(SwglDevice, f, names))
 
 
 @pytest.mark.parametrize("cam", PERSP_CAMERAS)
 @pytest.mark.parametrize("kind", ["solid", "solid_aa", "image", "image_nearest", "quad"])
-def test_perspective_brushes(kind, cam):
+def test_perspective_brushes(kind, cam, reference):
     """draw_perspective (rasterize.h:1422-1545): near-plane clipping, polygon edge walk, per-sample z and
     1/w-corrected varyings — byte-exact against SWGL."""
     d, ry, rx = cam
@@ -563,12 +563,13 @@ def test_perspective_brushes(kind, cam):
     else:
         f = scenes.perspective_frame("solid", d=d, ry=ry, rx=rx, seed=4 if kind == "solid_aa" else 3,
                                      force_aa=kind == "solid_aa", n_opaque=6, n_alpha=12)
-    assert_same(render(CudaDevice, f, ["target"]), render(_swgl(), f, ["target"]), f"{kind} {cam}")
+    want = _reference_pixels(reference, f, ["target"])
+    assert_same(render(CudaDevice, f, ["target"]), want, f"{kind} {cam}")
 
 
 @pytest.mark.parametrize("cam", PERSP_CAMERAS[:4])
 @pytest.mark.parametrize("kind", ["opacity", "blend", "mix_blend"])
-def test_perspective_picture_brushes(kind, cam):
+def test_perspective_picture_brushes(kind, cam, reference):
     """brush_opacity / brush_blend / brush_mix_blend drawing a picture's surface under a perspective node —
     byte-exact against SWGL (hue-rotate's cosf/sinf aside: <= 1 LSB, DESIGN.md section 4.4)."""
     d, ry, rx = cam
@@ -576,7 +577,8 @@ def test_perspective_picture_brushes(kind, cam):
     if kind == "opacity":
         kw.update(brush_flags=1)
     f = scenes.perspective_frame(kind, height=400 if kind != "opacity" else 360, d=d, ry=ry, rx=rx, **kw)
-    got, want = render(CudaDevice, f, ["target"]), render(_swgl(), f, ["target"])
+    want = _reference_pixels(reference, f, ["target"])
+    got = render(CudaDevice, f, ["target"])
     if kind == "blend":
         dd = np.abs(got["target"].astype(int) - want["target"].astype(int))
         assert dd.max() <= 1 and (dd != 0).mean() < 2e-3, (int(dd.max()), float((dd != 0).mean()))
@@ -584,19 +586,21 @@ def test_perspective_picture_brushes(kind, cam):
         assert_same(got, want, f"{kind} {cam}")
 
 
-def test_perspective_full_size():
+def test_perspective_full_size(reference):
     """4K: long polygon edges (rows up to 2160) and spans up to 3840 samples of stepped z/w."""
     f = scenes.perspective_frame("solid", width=3840, height=2160, d=3000.0, ry=50.0, rx=-20.0, seed=5, n_opaque=4,
                                  n_alpha=10, with_masks=False)
-    assert_same(render(CudaDevice, f, ["target"]), render(_swgl(), f, ["target"]))
+    want = _reference_pixels(reference, f, ["target"])
+    assert_same(render(CudaDevice, f, ["target"]), want)
 
 
 @pytest.mark.parametrize("kw", [dict(), dict(d=220.0, ry=65.0, rx=20.0), dict(perspective_interpolate=1, seed=3),
                                 dict(d=1e9, ry=0.0, rx=0.0, seed=4), dict(seed=5, filter=abi.NEAREST),
                                 dict(seed=6, width=1920, height=1080, n_polys=40, d=900.0)])
-def test_split_composite(kw):
+def test_split_composite(kw, reference):
     f = scenes.split_composite_frame(**kw)
-    assert_same(render(CudaDevice, f, ["target"]), render(_swgl(), f, ["target"]), str(kw))
+    want = _reference_pixels(reference, f, ["target"])
+    assert_same(render(CudaDevice, f, ["target"]), want, str(kw))
 
 
 @pytest.mark.parametrize("seed", [1, 2])

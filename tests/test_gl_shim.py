@@ -13,7 +13,7 @@ from oracle.backends import OracleDevice, SwglDevice
 from webrender_b200 import abi
 from workloads import scenes
 
-from common import assert_same, render
+from common import assert_same, reference, render  # noqa: F401 (reference: fixture)
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 GL_LIB = os.path.join(ROOT, "webrender_b200", "libwrcu_gl.so")
@@ -160,43 +160,46 @@ def run_sw_composite_yuv(dev, case, planes, via=None):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("case", SW_COMPOSITE_YUV_CASES, ids=[c[0] for c in SW_COMPOSITE_YUV_CASES])
-def test_sw_compositor_composite_yuv(case):
+def test_sw_compositor_composite_yuv(case, reference):
     """CompositeYUV (swgl/src/composite.h:1335-1384: linear_convert_yuv / linear_row_yuv / upscaleYUV42R8) through
     libwrcu_gl.so on the CUDA backend against the unmodified reference: 4:2:0, 4:2:2 and 4:4:4 planes, up- and
-    downscaling, flips, clips, sources partly outside the planes, every colour space — bytes equal."""
+    downscaling, flips, clips, sources partly outside the planes, every colour space — bytes equal.  The expected
+    bytes are the host emulation's, held to the digest of the reference build's output."""
+    from test_emu_parity import _emu_composite_yuv, _swgl_composite_yuv
     planes = sw_yuv_planes(case)
-    outs = []
-    for D in (GlShimDevice, SwglDevice):
-        d = D()
-        outs.append(run_sw_composite_yuv(d, case, planes))
-        d.close()
-    diff = outs[0] != outs[1]
+    want = reference(_emu_composite_yuv(case, planes), lambda: _swgl_composite_yuv(case, planes))["dst"]
+    d = GlShimDevice()
+    got = run_sw_composite_yuv(d, case, planes)
+    d.close()
+    diff = got != want
     assert not diff.any(), f"{int(diff.sum())} bytes differ, first at {np.argwhere(diff)[0]}"
-    assert (outs[0] != planes[3]).any()
+    assert (got != planes[3]).any()
 
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("case", SW_COMPOSITE_CASES, ids=[c[0] for c in SW_COMPOSITE_CASES])
-def test_sw_compositor_composite(case):
+def test_sw_compositor_composite(case, reference):
     """SwCompositor's hooks (LockTexture / Composite / GetResourceBuffer / UnlockResource,
     swgl/src/composite.h:485-590) on the CUDA backend against the unmodified reference: integer-ratio
-    nearest blits, 7-bit bilinear blits with their per-chunk running sums, flips, clips, over — bytes equal."""
+    nearest blits, 7-bit bilinear blits with their per-chunk running sums, flips, clips, over — bytes equal.
+    The expected bytes are the host emulation's, held to the digest of the reference build's output."""
+    from test_emu_parity import _emu_blit, _swgl_blit
     _, (sw, sh), sr, dr, opaque, fx, fy, lin, cr = case
     rng = np.random.RandomState(11)
     src = rng.randint(0, 256, (sh, sw, 4)).astype(np.uint8)
     a = src[..., 3:4].astype(np.uint16)
     src[..., :3] = (src[..., :3].astype(np.uint16) * a // 255).astype(np.uint8)
     dst = rng.randint(0, 256, (360, 640, 4)).astype(np.uint8)
-    outs = []
-    for D in (GlShimDevice, SwglDevice):
-        d = D()
-        ts = d.texture_create(abi.FMT_RGBA8, sw, sh)
-        td = d.texture_create(abi.FMT_RGBA8, 640, 360)
-        d.texture_upload(ts, 0, 0, sw, sh, src.reshape(sh, sw * 4))
-        d.texture_upload(td, 0, 0, 640, 360, dst.reshape(360, 640 * 4))
-        d.sw_composite(td, ts, sr, dr, opaque, fx, fy, lin, cr)
-        outs.append(d.locked_pixels(td))
-        d.close()
-    diff = outs[0] != outs[1]
+    call = (src, dst, sr, dr, opaque, fx, fy, lin, cr)
+    want = reference(_emu_blit(*call), lambda: _swgl_blit(*call))["dst"]
+    d = GlShimDevice()
+    ts = d.texture_create(abi.FMT_RGBA8, sw, sh)
+    td = d.texture_create(abi.FMT_RGBA8, 640, 360)
+    d.texture_upload(ts, 0, 0, sw, sh, src.reshape(sh, sw * 4))
+    d.texture_upload(td, 0, 0, 640, 360, dst.reshape(360, 640 * 4))
+    d.sw_composite(td, ts, sr, dr, opaque, fx, fy, lin, cr)
+    got = d.locked_pixels(td)
+    d.close()
+    diff = got != want
     assert not diff.any(), f"{int(diff.sum())} bytes differ, first at {np.argwhere(diff)[0]}"
-    assert (outs[0] != dst.reshape(360, 640 * 4)).any()
+    assert (got != dst.reshape(360, 640 * 4)).any()

@@ -1,7 +1,9 @@
 """Golden vectors produced by the reference itself (tests/golden/make_golden.py,
 from oracle/_ref = unmodified swgl/src/gl.cc): the oracle must reproduce them
 byte for byte on any box (CPU tier); the CUDA backend likewise (GPU tier)."""
+import io
 import json
+import lzma
 import os
 
 import numpy as np
@@ -14,6 +16,19 @@ from common import render
 
 HERE = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 INDEX = json.load(open(os.path.join(HERE, "index.json")))
+# the reference's own reftest images (wrench/reftests/<path>, all opaque, stored as RGB) and the rows of
+# image/yuv.png kept of them, as golden/make_reftest_images.py wrote them
+REFTEST_IMAGES = os.path.join(HERE, "reftest_images.npz.xz")
+YUV_ROWS = slice(10, 58)
+_reftest_images = []
+
+
+def reftest_image(path):
+    """wrench/reftests/<path> as int RGBA."""
+    if not _reftest_images:
+        _reftest_images.append(np.load(io.BytesIO(lzma.decompress(open(REFTEST_IMAGES, "rb").read()))))
+    rgb = _reftest_images[0][path]
+    return np.concatenate([rgb, np.full(rgb.shape[:2] + (1,), 255, np.uint8)], axis=2).astype(int)
 
 
 # cases whose CUDA result may differ from the reference by <= 1 LSB on a few
@@ -42,13 +57,8 @@ def _check(device_cls, name, tolerant=False):
 def test_config_a_against_reference_png():
     """Config A pinned on the reference's OWN golden image: the oracle's render of
     wrench/reftests/aa/rounded-rects.yaml against rounded-rects-ref.png under the
-    reftest's fuzz `fuzzy(1,1) fuzzy-if(platform(swgl),4,27)` (aa/reftest.list:1).
-    Needs /root/reference and PIL (this container); skipped elsewhere."""
-    png = "/root/reference/wrench/reftests/aa/rounded-rects-ref.png"
-    if not os.path.exists(png):
-        pytest.skip("reference tree not present")
-    Image = pytest.importorskip("PIL.Image")
-    ref = np.array(Image.open(png).convert("RGBA")).astype(int)
+    reftest's fuzz `fuzzy(1,1) fuzzy-if(platform(swgl),4,27)` (aa/reftest.list:1)."""
+    ref = reftest_image("aa/rounded-rects-ref.png")
     out = render(OracleDevice, scenes.config_a_frame(), ["target"])["target"].reshape(604, 1036, 4)
     rgba = out[..., [2, 1, 0, 3]].astype(int)
     d = np.abs(rgba - ref).max(axis=2)
@@ -83,11 +93,7 @@ def test_clip_reftests_against_reference_png(which, png, max_diff, max_px):
     """wrench/reftests/clip/{clip-mode,clip-ellipse}.yaml (Clip and ClipOut rounded /
     elliptical clips, incl. the frame builder's corner-overlap scaling) against the
     reference's own PNGs under the reftest's fuzz.  Measured: 0 differing pixels."""
-    path = "/root/reference/wrench/reftests/" + png
-    if not os.path.exists(path):
-        pytest.skip("reference tree not present")
-    Image = pytest.importorskip("PIL.Image")
-    ref = np.array(Image.open(path).convert("RGBA")).astype(int)
+    ref = reftest_image(png)
     f = scenes.reftest_clip_frame(which)
     d_ = f.textures["target"]
     out = render(OracleDevice, f, ["target"])["target"].reshape(d_.height, d_.width, 4)[..., [2, 1, 0, 3]].astype(int)
@@ -111,11 +117,7 @@ def test_box_shadow_reftests_against_reference_png(which, png, max_diff, max_px)
     (box_shadow.rs:341-401): the shadow colour as a Rectangle under a Clip and a ClipOut rounded-rect clip — inset
     (offset / spread) and outset — drawn the Indirect way with one ps_quad_mask per clip.  Against the reference's own
     PNGs under each reftest's fuzz."""
-    path = "/root/reference/wrench/reftests/" + png
-    if not os.path.exists(path):
-        pytest.skip("reference tree not present")
-    Image = pytest.importorskip("PIL.Image")
-    ref = np.array(Image.open(path).convert("RGBA")).astype(int)
+    ref = reftest_image(png)
     f = scenes.reftest_box_shadow_frame(which)
     d_ = f.textures["target"]
     out = render(OracleDevice, f, ["target"])["target"].reshape(d_.height, d_.width, 4)[..., [2, 1, 0, 3]].astype(int)
@@ -127,11 +129,7 @@ def test_box_shadow_reftests_against_reference_png(which, png, max_diff, max_px)
 def test_border_overlapping_reftest_against_reference_png():
     """wrench/reftests/border/overlapping.yaml == overlapping.png under fuzzy-if(platform(swgl),1,20): overlapping
     corner ellipses of a complex clip.  Measured: 0 pixels differ."""
-    path = "/root/reference/wrench/reftests/border/overlapping.png"
-    if not os.path.exists(path):
-        pytest.skip("reference tree not present")
-    Image = pytest.importorskip("PIL.Image")
-    ref = np.array(Image.open(path).convert("RGBA")).astype(int)
+    ref = reftest_image("border/overlapping.png")
     f = scenes.reftest_border_overlapping_frame()
     out = render(OracleDevice, f, ["target"])["target"].reshape(240, 233, 4)[..., [2, 1, 0, 3]].astype(int)
     d = np.abs(out - ref).max(axis=2)
@@ -142,11 +140,7 @@ def test_border_no_bogus_line_reftest_against_reference_png():
     """wrench/reftests/border/border-no-bogus-line.yaml == border-no-bogus-line-ref.png under
     fuzzy-if(platform(swgl),1,8): a rounded solid border whose radii are scaled to fit (corner tasks by cs_border_solid,
     segments by Brush(Image) from the texture cache).  Measured: 0 pixels differ."""
-    path = "/root/reference/wrench/reftests/border/border-no-bogus-line-ref.png"
-    if not os.path.exists(path):
-        pytest.skip("reference tree not present")
-    Image = pytest.importorskip("PIL.Image")
-    ref = np.array(Image.open(path).convert("RGBA")).astype(int)
+    ref = reftest_image("border/border-no-bogus-line-ref.png")
     f = scenes.reftest_border_no_bogus_line_frame()
     out = render(OracleDevice, f, ["target"])["target"].reshape(108, 116, 4)[..., [2, 1, 0, 3]].astype(int)
     d = np.abs(out - ref).max(axis=2)
@@ -159,11 +153,7 @@ def test_border_reftests_against_reference_png(name, png):
     """wrench/reftests/border/{border-radii,border-clamp-corner-radius}.yaml against the reference's images: solid
     rounded borders through the frame builder's segment decomposition (cs_border_solid corner and edge tasks in the
     texture cache, Brush(Image) per segment), per-corner radii and radii scaled to fit.  Measured: 0 pixels differ."""
-    path = "/root/reference/wrench/reftests/" + png
-    if not os.path.exists(path):
-        pytest.skip("reference tree not present")
-    Image = pytest.importorskip("PIL.Image")
-    ref = np.array(Image.open(path).convert("RGBA")).astype(int)
+    ref = reftest_image(png)
     (w, h), _, (max_diff, max_px) = scenes.BORDER_REFTESTS[name]
     assert ref.shape[:2] == (h, w)
     f = scenes.reftest_border_frame(name)
@@ -175,11 +165,7 @@ def test_border_reftests_against_reference_png(name, png):
 def test_clip_inverted_ellipse_reftest_against_reference_png():
     """wrench/reftests/clip/inverted-ellipse.yaml == inverted-ellipse.png (exact): an elliptical complex clip whose
     corner-size ratio is the inverse of the primitive's.  Measured: 0 pixels differ."""
-    path = "/root/reference/wrench/reftests/clip/inverted-ellipse.png"
-    if not os.path.exists(path):
-        pytest.skip("reference tree not present")
-    Image = pytest.importorskip("PIL.Image")
-    ref = np.array(Image.open(path).convert("RGBA")).astype(int)
+    ref = reftest_image("clip/inverted-ellipse.png")
     f = scenes.reftest_clip_inverted_ellipse_frame()
     out = render(OracleDevice, f, ["target"])["target"].reshape(236, 319, 4)[..., [2, 1, 0, 3]].astype(int)
     assert np.array_equal(out, ref), int((np.abs(out - ref).max(axis=2) > 0).sum())
@@ -189,20 +175,17 @@ def test_split_near_plane_reftest_against_reference_png():
     """wrench/reftests/split/near-plane.yaml == near-plane.png (fuzzy(1,20); fuzzy-if(platform(swgl),128,39)): one
     plane-split polygon crossing the near plane, drawn by ps_split_composite from the picture's surface — the
     perspective path (draw_perspective with frustum clipping, rasterize.h:1064-1545) against an image the reference's
-    authors checked in.  Drawn by the reference build (the plain-C port does not restate perspective); the same
-    bytes are a golden the emulated and the CUDA kernels must reproduce.  Measured: 0 pixels differ."""
-    path = "/root/reference/wrench/reftests/split/near-plane.png"
-    if not os.path.exists(path):
-        pytest.skip("reference tree not present")
-    Image = pytest.importorskip("PIL.Image")
-    from oracle.backends import SwglDevice
-    ref = np.array(Image.open(path).convert("RGBA")).astype(int)
+    authors checked in.  Drawn by the device code compiled for the host (the plain-C port does not restate
+    perspective), which must give the reference build's bytes (the stored golden).  Measured: 0 pixels differ."""
+    from emu import EmuDevice
+    ref = reftest_image("split/near-plane.png")
     f = scenes.reftest_split_near_plane_frame()
-    out = render(SwglDevice, f, ["target"])["target"].reshape(600, 600, 4)[..., [2, 1, 0, 3]].astype(int)
+    got = render(EmuDevice, f, ["target"])["target"]
+    out = got.reshape(600, 600, 4)[..., [2, 1, 0, 3]].astype(int)
     d = np.abs(out - ref).max(axis=2)
     assert d.max() <= 128 and int((d > 0).sum()) <= 39, (int(d.max()), int((d > 0).sum()))
     want = np.load(os.path.join(HERE, "reftest_split_near_plane.npz"))["target"]
-    assert np.array_equal(render(SwglDevice, f, ["target"])["target"], want)
+    assert np.array_equal(got, want)
 
 
 def _filter_reftest(device_cls, name):
@@ -264,11 +247,7 @@ def test_filter_blur_reftest_against_reference_png():
     filters/reftest.list:29): picture surface → vertical + horizontal cs_blur COLOR_TARGET → Brush(Image) composite,
     against the reference's own PNG.  Measured: max 2 on 10 744 pixels (52 of them at 2) — the blurred 6-pixel band
     around the square, where SWGL's 8-bit passes differ from the GL reference."""
-    path = "/root/reference/wrench/reftests/filters/filter-small-blur-radius.png"
-    if not os.path.exists(path):
-        pytest.skip("reference tree not present")
-    Image = pytest.importorskip("PIL.Image")
-    ref = np.array(Image.open(path).convert("RGBA")).astype(int)
+    ref = reftest_image("filters/filter-small-blur-radius.png")
     f = scenes.reftest_filter_blur_frame()
     out = render(OracleDevice, f, ["target"])["target"].reshape(700, 700, 4)[..., [2, 1, 0, 3]].astype(int)
     d = np.abs(out - ref).max(axis=2)
@@ -288,11 +267,7 @@ def test_filter_blur_reftest_against_reference_png():
 def test_gradient_reftests_against_reference_png(which, png, max_diff, max_px):
     """wrench/reftests/gradient/linear*.yaml as Brush(LinearGradient) against the
     reference's own PNGs under each reftest's fuzz (measured: 0 / 0 / <=1 on 4800 px)."""
-    path = "/root/reference/wrench/reftests/" + png
-    if not os.path.exists(path):
-        pytest.skip("reference tree not present")
-    Image = pytest.importorskip("PIL.Image")
-    ref = np.array(Image.open(path).convert("RGBA")).astype(int)
+    ref = reftest_image(png)
     out = render(OracleDevice, scenes.reftest_gradient_frame(which), ["target"])["target"]
     out = out.reshape(300, 300, 4)[..., [2, 1, 0, 3]].astype(int)
     h, w = min(ref.shape[0], 300), min(ref.shape[1], 300)
@@ -311,11 +286,7 @@ def test_cached_gradient_reftests_against_reference_png(which, png, max_diff, ma
     the frame builder draws them — a cached cs_radial_gradient / cs_conic_gradient render task in a
     texture-cache target, composited 1:1 with Brush(Image) — against the reference's OWN PNGs under each
     reftest's fuzz.  Pins the texture-cache-target gradient programs and the image composite."""
-    path = "/root/reference/wrench/reftests/" + png
-    if not os.path.exists(path):
-        pytest.skip("reference tree not present")
-    Image = pytest.importorskip("PIL.Image")
-    ref = np.array(Image.open(path).convert("RGBA")).astype(int)
+    ref = reftest_image(png)
     out = render(OracleDevice, scenes.reftest_cached_gradient_frame(which), ["target"])["target"]
     out = out.reshape(300, 300, 4)[..., [2, 1, 0, 3]].astype(int)
     d = np.abs(out - ref[:300, :300]).max(axis=2)
@@ -330,11 +301,7 @@ def test_more_cached_gradient_reftests_against_reference_png(name, png):
     """wrench/reftests/gradient/{radial-circle,radial-ellipse,conic-simple}.yaml against the reference's images under
     each reftest's own fuzz (1 on 80000 / 80000 / 300): cs_radial_gradient with ratio_xy != 1, cs_conic_gradient, 300x300
     tasks.  Measured: 1 LSB on 18 / 8 / 5 pixels."""
-    path = "/root/reference/wrench/reftests/" + png
-    if not os.path.exists(path):
-        pytest.skip("reference tree not present")
-    Image = pytest.importorskip("PIL.Image")
-    ref = np.array(Image.open(path).convert("RGBA")).astype(int)
+    ref = reftest_image(png)
     (w, h), _, _, _, _, _, (max_diff, max_px) = scenes.CACHED_GRADIENT_REFTESTS[name]
     f = scenes.reftest_cached_gradient_frame2(name)
     out = render(OracleDevice, f, ["target"])["target"].reshape(h, w, 4)[..., [2, 1, 0, 3]].astype(int)
@@ -347,11 +314,7 @@ def test_linear_aligned_border_radius_reftest_against_reference_png():
     GL; `==` there): vertical gradients under a rounded clip on white, blue and black — Brush(LinearGradient) alpha pass
     with cs_clip_rectangle masks.  Measured: 1 LSB on 231 of 59 645 pixels (the corner coverage and the gradient ramp
     round differently on GL); the reference build gives the same bytes as the port."""
-    path = "/root/reference/wrench/reftests/gradient/linear-aligned-border-radius.png"
-    if not os.path.exists(path):
-        pytest.skip("reference tree not present")
-    Image = pytest.importorskip("PIL.Image")
-    ref = np.array(Image.open(path).convert("RGBA")).astype(int)
+    ref = reftest_image("gradient/linear-aligned-border-radius.png")
     f = scenes.reftest_gradient_border_radius_frame()
     out = render(OracleDevice, f, ["target"])["target"].reshape(151, 395, 4)[..., [2, 1, 0, 3]].astype(int)
     d = np.abs(out - ref).max(axis=2)
@@ -362,11 +325,7 @@ def test_box_shadow_suite_through_the_compositor_against_reference_png():
     """The box-shadow suite drawn the way a page reaches the screen: into a picture-cache tile, then the tile list
     composited into the framebuffer (composite FAST_PATH, the copy class on the GPU) — the framebuffer against
     boxshadow/box-shadow-suite-no-blur.png: the same 1 LSB on 8 pixels as the direct draw."""
-    path = "/root/reference/wrench/reftests/boxshadow/box-shadow-suite-no-blur.png"
-    if not os.path.exists(path):
-        pytest.skip("reference tree not present")
-    Image = pytest.importorskip("PIL.Image")
-    ref = np.array(Image.open(path).convert("RGBA")).astype(int)
+    ref = reftest_image("boxshadow/box-shadow-suite-no-blur.png")
     f = scenes.reftest_box_shadow_suite_composited_frame()
     out = render(OracleDevice, f, ["fb"])["fb"].reshape(789, 894, 4)[..., [2, 1, 0, 3]].astype(int)
     d = np.abs(out - ref).max(axis=2)
@@ -377,11 +336,7 @@ def test_image_segments_reftest_against_reference_png():
     """wrench/reftests/image/segments.yaml == segments.png under fuzzy-if(platform(swgl),1,20): wrench's checkerboard
     image drawn 1:1 under a rounded clip (cs_clip_rectangle mask + Brush(Image) alpha pass) and unclipped (opaque
     Brush(Image)).  Measured: 1 LSB on 18 pixels."""
-    path = "/root/reference/wrench/reftests/image/segments.png"
-    if not os.path.exists(path):
-        pytest.skip("reference tree not present")
-    Image = pytest.importorskip("PIL.Image")
-    ref = np.array(Image.open(path).convert("RGBA")).astype(int)
+    ref = reftest_image("image/segments.png")
     f = scenes.reftest_image_segments_frame()
     out = render(OracleDevice, f, ["target"])["target"].reshape(583, 290, 4)[..., [2, 1, 0, 3]].astype(int)
     d = np.abs(out - ref).max(axis=2)
@@ -393,11 +348,7 @@ def test_line_decorations_reftest_against_reference_png():
     columns 0-217) of decorations-suite.png: solid, dashed, dotted and wavy lines at two thicknesses — cs_line_decoration
     tasks repeated along the line by Brush(Image) REPETITION.  The reftest allows SWGL 3 on 13 540 pixels over the whole
     suite; measured on this region: 0 pixels differ (2 001 of its 21 800 pixels are drawn)."""
-    path = "/root/reference/wrench/reftests/text/decorations-suite.png"
-    if not os.path.exists(path):
-        pytest.skip("reference tree not present")
-    Image = pytest.importorskip("PIL.Image")
-    ref = np.array(Image.open(path).convert("RGBA")).astype(int)
+    ref = reftest_image("text/decorations-suite.png")
     f = scenes.reftest_line_decorations_frame()
     out = render(OracleDevice, f, ["target"])["target"].reshape(439, 495, 4)[..., [2, 1, 0, 3]].astype(int)
     assert np.array_equal(out[:100, :218], ref[:100, :218])
@@ -409,13 +360,11 @@ def test_yuv_reftest_against_reference_png():
     from the reference's own plane PNGs) drawn as the frame builder draws it — opaque Brush(YuvImage)
     primitives into 1024x512 picture-cache tiles, tiles composited — against the reference's OWN yuv.png.
     The reference's annotation for SWGL on this content is fuzzy(1,205000) (image/reftest.list:9, the
-    brush path; 8-bit fixed-point YUV matrix vs the GPU's float one): measured max 1 on 204390 pixels."""
-    path = "/root/reference/wrench/reftests/image/yuv.png"
-    if not os.path.exists(path):
-        pytest.skip("reference tree not present")
-    Image = pytest.importorskip("PIL.Image")
-    ref = np.array(Image.open(path).convert("RGBA")).astype(int)
-    out = render(OracleDevice, scenes.reftest_yuv_frame(), ["target"])["target"]
-    out = out.reshape(658, 1323, 4)[..., [2, 1, 0, 3]].astype(int)
+    brush path; 8-bit fixed-point YUV matrix vs the GPU's float one): measured max 1 on 204390 pixels of the
+    whole page.  The planes are stored for their first rows only (golden/reftest_yuv), so the page is
+    compared on the rows those draw (YUV_ROWS, 1:1 from y = 10), under the same fuzz: max 1 on 24469 of them."""
+    ref = reftest_image("image/yuv.png")
+    out = render(OracleDevice, scenes.reftest_yuv_frame(os.path.join(HERE, "reftest_yuv")), ["target"])["target"]
+    out = out.reshape(658, 1323, 4)[YUV_ROWS, :, [2, 1, 0, 3]].astype(int)
     d = np.abs(out - ref).max(axis=2)
     assert d.max() <= 1 and int((d > 0).sum()) <= 205000, (int(d.max()), int((d > 0).sum()))

@@ -4,7 +4,9 @@ SWGL, the oracle, the host emulation and (GPU tier) the CUDA backend."""
 import numpy as np
 import pytest
 
-from oracle.backends import OracleDevice, SwglDevice, have_swgl
+from oracle.backends import OracleDevice, SwglDevice
+
+from common import reference  # noqa: F401 (fixture)
 
 from update_path import run_sequence
 
@@ -17,15 +19,13 @@ def _run(cls, kind, seed):
         dev.close()
 
 
-@pytest.mark.skipif(not have_swgl(), reason="oracle/_ref not built (needs /root/reference)")
 @pytest.mark.parametrize("kind", ["text", "image"])
 @pytest.mark.parametrize("seed", [1, 2])
-def test_oracle_matches_reference_plumbing(kind, seed):
-    a = _run(SwglDevice, kind, seed)
-    b = _run(OracleDevice, kind, seed)
-    for x, y in zip(a, b):
-        assert np.array_equal(x, y)
-    assert not np.array_equal(a[0], a[1])   # frame 2 really differs (patched cache / moved tile)
+def test_oracle_matches_reference_plumbing(kind, seed, reference):
+    def frames(cls):
+        return {f"frame{i}": x for i, x in enumerate(_run(cls, kind, seed))}
+    b = reference(frames(OracleDevice), lambda: frames(SwglDevice))
+    assert not np.array_equal(b["frame0"], b["frame1"])   # frame 2 really differs (patched cache / moved tile)
 
 
 @pytest.mark.parametrize("kind", ["text", "image"])

@@ -1757,12 +1757,13 @@ def yuv_image_frame(fmt="planar", color_space=2, seed=1, width=512, height=320, 
     return Frame(t.arrays(), textures, [[Target("target", ops=ops)]])
 
 
-def reftest_yuv_frame(ref_dir="/root/reference/wrench/reftests/image"):
+def reftest_yuv_frame(ref_dir):
     """wrench/reftests/image/yuv.yaml the way the frame builder draws it: three `yuv-image` items of 427x640 at
     1:1 — planar (three R8 planes), interleaved (one BGRA image: Cb, Y, Cr in B, G, R) and NV12 with the CbCr
     plane loaded as a BGRA image (wrench turns RGB PNGs into BGRA8: Cb in R, Cr in G — sampleYUV's RGBA8 branch,
     swgl_ext.h:1069-1075) — Color8, Rec709, limited range (yaml_frame_reader.rs:1203-1206), as opaque
-    Brush(YuvImage) primitives on the white 1323x658 page.  Reads the reference's own plane PNGs."""
+    Brush(YuvImage) primitives on the white 1323x658 page.  Reads the reference's own plane PNGs from `ref_dir`
+    (wrench/reftests/image of a WebRender checkout)."""
     from PIL import Image
     from webrender_b200.gpu_types import brush_instance, CLIP_TASK_EMPTY, YUV_FORMAT_PLANAR, YUV_FORMAT_NV12, YUV_FORMAT_INTERLEAVED
     import os
