@@ -62,8 +62,12 @@ typedef enum wrcu_format {
   WRCU_FMT_RGBAF32 = 3, /* 16 B/texel (data textures, GPU cache)          */
   WRCU_FMT_RGBAI32 = 4, /* 16 B/texel                                     */
   WRCU_FMT_DEPTH24 = 5, /* 4 B/px, 24-bit depth (rasterize.h:37)          */
-  WRCU_FMT_RG8 = 6      /* 2 B/px, sample-only: the CbCr plane of NV12 video
+  WRCU_FMT_RG8 = 6,     /* 2 B/px, sample-only: the CbCr plane of NV12 video
                            surfaces (gl.cc:247, TextureFormat::RG8)          */
+  WRCU_FMT_R16 = 7,     /* 2 B/px, sample-only: a 10/12/16-bit video plane
+                           (gl.cc:257, TextureFormat::R16)                   */
+  WRCU_FMT_RG16 = 8     /* 4 B/px, sample-only: the CbCr plane of 10/12/16-bit
+                           NV12 and P010 surfaces (gl.cc:259, TextureFormat::RG16) */
 } wrcu_format;
 
 typedef enum wrcu_filter { WRCU_NEAREST = 0, WRCU_LINEAR = 1 } wrcu_filter;
@@ -115,7 +119,9 @@ enum {
   WRCU_FEAT_ALPHA_TARGET = 1u << 8, /* cs_blur into an R8 target    */
   WRCU_FEAT_COLOR_TARGET = 1u << 9, /* cs_blur into an RGBA8 target */
   WRCU_FEAT_YUV = 1u << 10          /* composite: YUV video surfaces (composite.glsl:14-33),
-                                       8-bit PLANAR / NV12 / INTERLEAVED planes    */
+                                       8-bit PLANAR / NV12 / INTERLEAVED planes;
+                                       10/12/16-bit PLANAR (3 x R16), NV12 and P010
+                                       (R16 + RG16)                                */
 };
 
 /* Blend keys: exactly the set the reference's blend stage implements
@@ -342,12 +348,14 @@ int wrcu_composite_blit(wrcu_ctx* ctx, wrcu_tex dst, wrcu_tex src,
                         const int32_t clip_rect[4]);
 
 /* `CompositeYUV` of the SWGL surface (swgl/src/composite.h:1335-1384; compositor/sw_compositor.rs composites video
- * surfaces with it): three 8-bit planes (R8 textures; the two chroma planes of one size, full or half resolution)
+ * surfaces with it): three planes (R8 textures at `color_depth` 8, or LSB-aligned R16 textures at `color_depth`
+ * 10, 12 or 16; the two chroma planes of one size, full or half resolution)
  * converted to BGRA with the 6/7-bit fixed-point matrix of `color_space` (YUVRangedColorSpace, composite.h:1210-1218:
  * 0 BT601 narrow, 1 BT601 full, 2 BT709 narrow, 3 BT709 full, 4 BT2020 narrow, 5 BT2020 full, 6 GBR identity) while the
  * `src_rect` of the luma plane is scaled into `dst_rect` with the reference's row walker (linear_row_yuv: integer
- * coordinates, the half-resolution-chroma upscale path included), clipped to `clip_rect`; opaque.  Bit-exact.
- * `color_depth` must be 8 (R16 planes: WRCU_ERR_UNSUPPORTED, as are planes under 2 texels wide). */
+ * coordinates, the half-resolution-chroma upscale path of 8-bit planes included), clipped to `clip_rect`; opaque.
+ * Bit-exact.  The matrix is the 8-bit one at every depth, as in the reference.  Any other plane format / depth
+ * combination, and planes under 2 texels wide, give WRCU_ERR_UNSUPPORTED. */
 int wrcu_composite_blit_yuv(wrcu_ctx* ctx, wrcu_tex dst, wrcu_tex y_plane, wrcu_tex u_plane, wrcu_tex v_plane,
                             int color_space, uint32_t color_depth,
                             const int32_t src_rect[4], const int32_t dst_rect[4],

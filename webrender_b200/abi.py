@@ -11,8 +11,9 @@ ABI_VERSION = 1
 OK, ERR_INVALID, ERR_OOM, ERR_CUDA, ERR_UNSUPPORTED, ERR_NO_DEVICE = 0, -1, -2, -3, -4, -5
 
 # wrcu_format
-FMT_RGBA8, FMT_R8, FMT_RGBAF32, FMT_RGBAI32, FMT_DEPTH24, FMT_RG8 = 1, 2, 3, 4, 5, 6
-FMT_BPP = {FMT_RGBA8: 4, FMT_R8: 1, FMT_RGBAF32: 16, FMT_RGBAI32: 16, FMT_DEPTH24: 4, FMT_RG8: 2}
+FMT_RGBA8, FMT_R8, FMT_RGBAF32, FMT_RGBAI32, FMT_DEPTH24, FMT_RG8, FMT_R16, FMT_RG16 = 1, 2, 3, 4, 5, 6, 7, 8
+FMT_BPP = {FMT_RGBA8: 4, FMT_R8: 1, FMT_RGBAF32: 16, FMT_RGBAI32: 16, FMT_DEPTH24: 4, FMT_RG8: 2, FMT_R16: 2,
+           FMT_RG16: 4}
 
 NEAREST, LINEAR = 0, 1
 

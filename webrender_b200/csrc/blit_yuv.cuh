@@ -8,6 +8,8 @@
 // Every quantity of chunk n is a closed form of n (the coordinates advance by integer additions), so a
 // THREAD takes a (row, chunk) and reproduces the reference's lanes for it; the host computes the
 // row-invariant start lanes and the phase boundaries with the reference's own float and integer steps.
+// 10-, 12- and 16-bit planes (R16 textures, colorDepth > 8) take one phase: every chunk goes through
+// textureLinearUnpackedR16 >> (colorDepth - 1 - 8) (composite.h:1025-1058), with the same 8-bit matrix.
 #pragma once
 #include "shader_composite_yuv.cuh"
 
@@ -24,6 +26,7 @@ struct YuvBlitArgs {
   int fast;              // the half-resolution fast path's condition holds
   int pre, inside;       // chunks before the upscale phase, pixels inside it
   int color_space;       // YUVRangedColorSpace (composite.h:1210-1218): same numbering as yuv.glsl's
+  int rescale_bits;      // R16 planes: colorDepth - 1 - 8
 };
 
 WRD int wr_yb_clamp(int v, int lo, int hi) { return v < lo ? lo : (v > hi ? hi : v); }
@@ -118,11 +121,31 @@ WRD void wr_yuv_blit_chunk(const YuvBlitArgs& a, const YuvFixed& fm, int r, int 
   for (int j = 0; j < cnt; j++) d[j] = wr_yb_pack(wr_yuv_convert(fm, Y[j], U[j], V[j]));
 }
 
+// chunk n of row r, R16 planes (linear_row_yuv's R16 branch, composite.h:1025-1058)
+WRD void wr_yuv_blit_chunk16(const YuvBlitArgs& a, const YuvFixed& fm, int r, int n) {
+  const int yV = (int)wr_repeat_add(a.v0, a.dv, r), cV = (int)wr_repeat_add(a.cv0, a.cdv, r);
+  uint32_t* d = (uint32_t*)(a.dst + (size_t)(a.dy + r) * a.dst_pitch) + a.dx + 4 * n;
+  const int cnt = min(4, a.span - 4 * n);
+  for (int j = 0; j < cnt; j++) {
+    const int yq = (a.yU0[j] + n * a.yDU) >> WR_YUV_STEP_BITS, cq = (a.cU0[j] + n * a.cDU) >> WR_YUV_STEP_BITS;
+    int Y, U, V;
+    wr_texture_linear_16(a.yp, a.y_pitch, a.yw, a.yh, 1, yq, yV, &Y);
+    wr_texture_linear_16(a.up, a.c_pitch, a.cw, a.ch, 1, cq, cV, &U);
+    wr_texture_linear_16(a.vp, a.c_pitch, a.cw, a.ch, 1, cq, cV, &V);
+    d[j] = wr_yb_pack(wr_yuv_convert(fm, Y >> a.rescale_bits, U >> a.rescale_bits, V >> a.rescale_bits));
+  }
+}
+
 #ifdef WRCU_HOSTEMU
 static void wr_sw_composite_blit_yuv(YuvBlitArgs a) {
   const YuvFixed fm = wr_yuv_blit_matrix(a.color_space);
   for (int r = 0; r < a.rows; r++)
     for (int n = 0; 4 * n < a.span; n++) wr_yuv_blit_chunk(a, fm, r, n);
+}
+static void wr_sw_composite_blit_yuv16(YuvBlitArgs a) {
+  const YuvFixed fm = wr_yuv_blit_matrix(a.color_space);
+  for (int r = 0; r < a.rows; r++)
+    for (int n = 0; 4 * n < a.span; n++) wr_yuv_blit_chunk16(a, fm, r, n);
 }
 #else
 __global__ void wr_sw_composite_blit_yuv(YuvBlitArgs a) {
@@ -131,5 +154,12 @@ __global__ void wr_sw_composite_blit_yuv(YuvBlitArgs a) {
   __syncthreads();
   const int n = blockIdx.x * blockDim.x + threadIdx.x, r = blockIdx.y * blockDim.y + threadIdx.y;
   if (4 * n < a.span && r < a.rows) wr_yuv_blit_chunk(a, fm, r, n);
+}
+__global__ void wr_sw_composite_blit_yuv16(YuvBlitArgs a) {
+  __shared__ YuvFixed fm;
+  if (threadIdx.x == 0 && threadIdx.y == 0) fm = wr_yuv_blit_matrix(a.color_space);
+  __syncthreads();
+  const int n = blockIdx.x * blockDim.x + threadIdx.x, r = blockIdx.y * blockDim.y + threadIdx.y;
+  if (4 * n < a.span && r < a.rows) wr_yuv_blit_chunk16(a, fm, r, n);
 }
 #endif

@@ -1,7 +1,8 @@
 // shader_composite_yuv.cuh — composite with WR_FEATURE_YUV (webrender/res/composite.glsl:14-33,
 // 83-130, 163-176, 197-214 + webrender/res/yuv.glsl): external video surfaces converted
 // YCbCr → RGB while they are composited.  8-bit planes: PLANAR (three R8 textures), NV12
-// (R8 + RG8 or RGBA8) and INTERLEAVED (one BGRA texture).
+// (R8 + RG8 or RGBA8) and INTERLEAVED (one BGRA texture); 10-, 12- and 16-bit planes: PLANAR (three
+// R16 textures) and NV12 / P010 (R16 + RG16), LSB-aligned except P010 (see wr_yuv_rescale).
 //
 // Span body (len & ~3): swgl_commitTextureLinearYUV → blendYUV → blendYUVFallback
 // (swgl/src/swgl_ext.h:1006-1187): every plane is sampled through the fallback bilinear filter
@@ -31,8 +32,59 @@ WRD void wr_texture_linear_rg8(const TexView& t, int ix, int iy, int* out) {
   }
 }
 
-// texture() of the fragment path for the plane formats (adds RG8 to wr_tex_fragment)
+// a + (((b - a) * f) >> 16) << 1 in int16 lanes: the 15-bit lerp of the R16 / RG16 fetches in the generic
+// (non-SSE) build (texture.h:680-700); f is the 7-bit fraction shifted left by 8
+WRD int wr_lerp15(int a, int b, int f) {
+  const int d = (int)(short)(b - a);
+  return (int)(short)(a + (int)(short)((int)(short)((d * f) >> 16) << 1));
+}
+// textureLinearUnpackedR16 / textureLinearUnpackedRG16 for one lane (texture.h:650-830): `nch` 16-bit channels
+// per texel, each shifted right by one into a signed 15-bit sample.  The x fraction is computed inline, not by
+// computeFracX: past the last column pair it is 127/128, not 128/128.
+WRD void wr_texture_linear_16(const uint8_t* base, int pitch, int w, int h, int nch, int ix, int iy, int* out) {
+  const int x = ix >> 7, y = iy >> 7;
+  const int cx = wr_clamp_coord(x, w - 1), cy = wr_clamp_coord(y, h);
+  const uint16_t* row0 = (const uint16_t*)(base + (size_t)cy * pitch) + (size_t)cx * nch;
+  const uint16_t* row1 = (const uint16_t*)((const uint8_t*)row0 + ((y >= 0 && y < h - 1) ? pitch : 0));
+  const int fx = (((ix & (x >= 0 ? -1 : 0)) | (x > w - 2 ? -1 : 0)) & 0x7F) << 8;
+  const int fy = (iy & 0x7F) << 8;
+  for (int ch = 0; ch < nch; ch++) {
+    const int a0 = __ldg(row0 + ch) >> 1, a1 = __ldg(row1 + ch) >> 1;
+    const int b0 = __ldg(row0 + nch + ch) >> 1, b1 = __ldg(row1 + nch + ch) >> 1;
+    out[ch] = wr_lerp15(wr_lerp15(a0, a1, fy), wr_lerp15(b0, b1, fy), fx);
+  }
+}
+WRD int wr_texture_linear_r16(const TexView& t, int ix, int iy) {
+  int v;
+  wr_texture_linear_16(t.ptr, t.pitch, t.w, t.h, 1, ix, iy, &v);
+  return v;
+}
+
+// texture() of the fragment path for the plane formats (adds RG8 to wr_tex_fragment; HDR: R16 and RG16 only)
+template <bool HDR>
 WRD void wr_yuv_tex_fragment(const TexView& t, float cu, float cv, float* out) {
+  if (HDR) {
+    const int nch = t.fmt == WRCU_FMT_R16 ? 1 : 2;
+    float s[2] = {0.0f, 0.0f};
+    if (t.filter == WRCU_LINEAR) {
+      // textureLinearR16 / textureLinearRG16 (texture.h:723-729, 823-830): int15 / 32767; RG16's red channel is
+      // read back as the unsigned low half of its 32-bit lane
+      int v[2];
+      wr_texture_linear_16(t.ptr, t.pitch, t.w, t.h, nch, (int)wr_linear_quantize(cu, t.w), (int)wr_linear_quantize(cv, t.h), v);
+      s[0] = (float)(nch == 2 ? (v[0] & 0xFFFF) : v[0]) * (1.0f / 32767.0f);
+      if (nch == 2) s[1] = (float)v[1] * (1.0f / 32767.0f);
+    } else {
+      // texelFetchR16 / texelFetchRG16 (texture.h:149-176): u16 / 65535
+      int x = wr_clamp_coord((int)(cu * (float)t.w), t.w), y = wr_clamp_coord((int)(cv * (float)t.h), t.h);
+      const uint16_t* p = (const uint16_t*)(t.ptr + (size_t)y * t.pitch) + (size_t)x * nch;
+      for (int ch = 0; ch < nch; ch++) s[ch] = (float)__ldg(p + ch) * (1.0f / 65535.0f);
+    }
+    out[0] = s[0];
+    out[1] = s[1];
+    out[2] = 0.0f;
+    out[3] = 1.0f;
+    return;
+  }
   if (t.fmt != WRCU_FMT_RG8) {
     wr_tex_fragment(t, cu, cv, out);
     return;
@@ -72,9 +124,12 @@ WRD Px wr_yuv_convert(const YuvFixed& m, int y, int u, int v) {
   return Px{wr_yuv_pack8(b), wr_yuv_pack8(g), wr_yuv_pack8(r), 255};
 }
 
+// One shader, two kernels: HDR = false samples the 8-bit plane sets, HDR = true the 16-bit ones (R16 luma; the
+// launch picks it from the luma plane's format), so the 8-bit kernel carries none of the 16-bit code.
 // CmdCold: g[0..11] vUVBounds_y/u/v, g[12..14] vYcbcrBias, g[15..23] vRgbFromDebiasedYcbcr
 // (column-major), g[24..31] YuvFixed (int bits), g[32] != 0: clamp rgb (brush_yuv_image ALPHA_PASS,
-// yuv.glsl:239-243); i[0] = vYuvFormat.x, i[1] = planes, i[2..3] the u chain table
+// yuv.glsl:239-243), g[33] (int bits) rescaleBits of 16-bit planes; i[0] = vYuvFormat.x, i[1] = planes,
+// i[2..3] the u chain table
 struct CompositeYuvShader {
   struct PlaneRow {
     float bu[4], bv[4];  // quantised uv lanes of chunk kb
@@ -91,7 +146,8 @@ struct CompositeYuvShader {
   WRD_MEMBER const TexView& plane(const RasterArgs& a, int p) {
     return p == 0 ? a.color0 : (p == 1 ? a.color1 : a.color2);
   }
-  WRD_MEMBER void row_setup(const RasterArgs& a, const CmdHot& c, int y, int tx0, bool rgba, Row& r) {
+  template <bool HDR>
+  WRD_MEMBER void row_setup_t(const RasterArgs& a, const CmdHot& c, int y, int tx0, bool rgba, Row& r) {
     const CmdCold& k = a.cold[c.cold];
     wr_row_interp<6>(a, k, c, y, r.o, r.step);
     int len = c.x1 - c.x0;
@@ -99,7 +155,9 @@ struct CompositeYuvShader {
     bool ok = rgba && len >= 4;
     for (int p = 0; p < planes; p++) ok = ok && plane(a, p).filter == WRCU_LINEAR;
     // sampleYUV's format switches (swgl_ext.h:1009-1127)
-    if (planes == 3) ok = ok && a.color0.fmt == WRCU_FMT_R8 && a.color1.fmt == WRCU_FMT_R8 && a.color2.fmt == WRCU_FMT_R8;
+    if (HDR) ok = ok && (planes == 3 ? a.color1.fmt == WRCU_FMT_R16 && a.color2.fmt == WRCU_FMT_R16
+                                     : planes == 2 && a.color1.fmt == WRCU_FMT_RG16);
+    else if (planes == 3) ok = ok && a.color0.fmt == WRCU_FMT_R8 && a.color1.fmt == WRCU_FMT_R8 && a.color2.fmt == WRCU_FMT_R8;
     else if (planes == 2) ok = ok && a.color0.fmt == WRCU_FMT_R8 && (a.color1.fmt == WRCU_FMT_RG8 || a.color1.fmt == WRCU_FMT_RGBA8);
     else ok = ok && a.color0.fmt == WRCU_FMT_RGBA8;
     r.body_len = ok ? (len & ~3) : 0;
@@ -182,7 +240,8 @@ struct CompositeYuvShader {
     for (int p = 0; p < 3; p++)
       r.p[p].exact = (wr_sum_exact(r.p[p].bu, r.p[p].ustep) ? 1 : 0) | (wr_sum_exact(r.p[p].bv, r.p[p].vstep) ? 2 : 0);
   }
-  WRD_MEMBER Px source(const RasterArgs& a, const CmdHot& c, const Row& r, int x, int, bool) {
+  template <bool HDR>
+  WRD_MEMBER Px source_t(const RasterArgs& a, const CmdHot& c, const Row& r, int x) {
     const CmdCold& k = a.cold[c.cold];
     int rel = x - c.x0;
     const int planes = k.i[1], format = k.i[0];
@@ -205,7 +264,19 @@ struct CompositeYuvShader {
         ii[p][1] = (int)wr_clamp(qv, pr.minv, pr.maxv);
       }
       int yv, uu, vv;
-      if (planes == 3) {
+      if (HDR) {
+        // 16-bit planes (swgl_ext.h:1078-1093, 1124-1140): 15-bit samples shifted down by rescaleBits
+        const int rb = ((const int*)k.g)[33];
+        yv = wr_texture_linear_r16(a.color0, ii[0][0], ii[0][1]) >> rb;
+        if (planes == 3) {
+          uu = wr_texture_linear_r16(a.color1, ii[1][0], ii[1][1]) >> rb;
+          vv = wr_texture_linear_r16(a.color2, ii[2][0], ii[2][1]) >> rb;
+        } else {
+          int uv[2];
+          wr_texture_linear_16(a.color1.ptr, a.color1.pitch, a.color1.w, a.color1.h, 2, ii[1][0], ii[1][1], uv);
+          uu = uv[0] >> rb; vv = uv[1] >> rb;
+        }
+      } else if (planes == 3) {
         yv = wr_texture_linear_r8(a.color0, ii[0][0], ii[0][1]);
         uu = wr_texture_linear_r8(a.color1, ii[1][0], ii[1][1]);
         vv = wr_texture_linear_r8(a.color2, ii[2][0], ii[2][1]);
@@ -250,14 +321,14 @@ struct CompositeYuvShader {
     }
     float s3[3] = {0.0f, 0.0f, 0.0f}, t4[4];
     if (format == 3) {
-      wr_yuv_tex_fragment(a.color0, cc[0][0], cc[0][1], t4); s3[0] = t4[0];
-      wr_yuv_tex_fragment(a.color1, cc[1][0], cc[1][1], t4); s3[1] = t4[0];
-      wr_yuv_tex_fragment(a.color2, cc[2][0], cc[2][1], t4); s3[2] = t4[0];
+      wr_yuv_tex_fragment<HDR>(a.color0, cc[0][0], cc[0][1], t4); s3[0] = t4[0];
+      wr_yuv_tex_fragment<HDR>(a.color1, cc[1][0], cc[1][1], t4); s3[1] = t4[0];
+      wr_yuv_tex_fragment<HDR>(a.color2, cc[2][0], cc[2][1], t4); s3[2] = t4[0];
     } else if (format >= 0 && format <= 2) {
-      wr_yuv_tex_fragment(a.color0, cc[0][0], cc[0][1], t4); s3[0] = t4[0];
-      wr_yuv_tex_fragment(a.color1, cc[1][0], cc[1][1], t4); s3[1] = t4[0]; s3[2] = t4[1];
+      wr_yuv_tex_fragment<HDR>(a.color0, cc[0][0], cc[0][1], t4); s3[0] = t4[0];
+      wr_yuv_tex_fragment<HDR>(a.color1, cc[1][0], cc[1][1], t4); s3[1] = t4[0]; s3[2] = t4[1];
     } else if (format == 4) {
-      wr_yuv_tex_fragment(a.color0, cc[0][0], cc[0][1], t4); s3[0] = t4[1]; s3[1] = t4[2]; s3[2] = t4[0];
+      wr_yuv_tex_fragment<HDR>(a.color0, cc[0][0], cc[0][1], t4); s3[0] = t4[1]; s3[1] = t4[2]; s3[2] = t4[0];
     }
     float dv[3] = {s3[0] - k.g[12], s3[1] - k.g[13], s3[2] - k.g[14]};
     float col[3];
@@ -272,6 +343,16 @@ struct CompositeYuvShader {
     o.a = 255;
     return o;
   }
+  WRD_MEMBER void row_setup(const RasterArgs& a, const CmdHot& c, int y, int tx0, bool rgba, Row& r) {
+    row_setup_t<false>(a, c, y, tx0, rgba, r);
+  }
+  WRD_MEMBER Px source(const RasterArgs& a, const CmdHot& c, const Row& r, int x, int, bool) { return source_t<false>(a, c, r, x); }
+};
+struct CompositeYuv16Shader : CompositeYuvShader {
+  WRD_MEMBER void row_setup(const RasterArgs& a, const CmdHot& c, int y, int tx0, bool rgba, Row& r) {
+    row_setup_t<true>(a, c, y, tx0, rgba, r);
+  }
+  WRD_MEMBER Px source(const RasterArgs& a, const CmdHot& c, const Row& r, int x, int, bool) { return source_t<true>(a, c, r, x); }
 };
 
 // get_yuv_color_info + get_rgb_from_ycbcr_info (yuv.glsl:79-161); m is column-major [col*3+row]
@@ -406,6 +487,42 @@ WRD void wr_yuv_chain_table(const SetupArgs& a, int idx, int planes, const TexVi
 #endif
 }
 
+// The plane sets the span and fragment stages sample (sampleYUV's format switches, swgl_ext.h:1009-1140):
+// depth 8 keeps the 8-bit sets (no 16-bit plane, no P010); depth 10, 12 or 16 takes three R16 planes (PLANAR) or
+// R16 + RG16 (NV12, P010).  Returns vRescaleFactor (composite.glsl:90-96: 16 - depth for the LSB-aligned formats,
+// 0 for MSB-aligned P010), or -1 for any other combination.
+WRD int wr_yuv_planes(int format) { return format == 3 ? 3 : (format == 0 || format == 1 ? 2 : (format == 4 ? 1 : 0)); }
+WRD int wr_yuv_rescale(int format, int bit_depth, const TexView* const* tv) {
+  if (bit_depth == 8) {
+    if (format == 1) return -1;
+    for (int p = 0; p < wr_yuv_planes(format); p++)
+      if (tv[p]->fmt == WRCU_FMT_R16 || tv[p]->fmt == WRCU_FMT_RG16) return -1;
+    return 0;
+  }
+  if (bit_depth != 10 && bit_depth != 12 && bit_depth != 16) return -1;
+  if (format == 3) {
+    if (tv[0]->fmt != WRCU_FMT_R16 || tv[1]->fmt != WRCU_FMT_R16 || tv[2]->fmt != WRCU_FMT_R16) return -1;
+  } else if (format == 0 || format == 1) {
+    if (tv[0]->fmt != WRCU_FMT_R16 || tv[1]->fmt != WRCU_FMT_RG16) return -1;
+  } else {
+    return -1;
+  }
+  return format == 1 ? 0 : 16 - bit_depth;
+}
+
+// An instance that is not drawn: an empty command with wr_emit_quad's cold record for a culled quad — the warp-wide
+// row-table and chain fills after the vertex stage read every instance's record, which must not be a stale one.
+WRD void wr_yuv_reject(const SetupArgs& a, int idx) {
+  CmdHot h = CmdHot{};
+  h.cold = idx;
+  a.hot[idx] = h;
+  CmdCold& k = a.cold[idx];
+  k.row_off = -1;
+  k.row_n = 0;
+  k.fail_off = -1;
+  k.i[2] = -1;
+}
+
 // composite vertex stage, YUV branch (composite.glsl:73-130)
 WRD void wr_setup_composite_yuv_one(const SetupArgs& a, int idx) {
   const float* f = (const float*)(a.instances + (size_t)idx * a.stride);
@@ -417,12 +534,13 @@ WRD void wr_setup_composite_yuv_one(const SetupArgs& a, int idx) {
   float rect[4] = {(dr[2] - dr[0]) * flipx + dr[0], (dr[3] - dr[1]) * flipy + dr[1],
                    (dr[0] - dr[2]) * flipx + dr[2], (dr[1] - dr[3]) * flipy + dr[3]};
   int color_space = (int)f[13], format = (int)f[14], bit_depth = (int)f[15];
-  int planes = format == 3 ? 3 : (format == 0 ? 2 : (format == 4 ? 1 : 0));
+  int planes = wr_yuv_planes(format);
   const TexView* tv[3] = {&a.color0, &a.color1, &a.color2};
-  bool bad = bit_depth != 8 || planes == 0;  // 10/12/16-bit planes (R16/RG16, P010) are not built
+  const int rescale = wr_yuv_rescale(format, bit_depth, tv);
+  bool bad = rescale < 0 || planes == 0;
   for (int p = 0; p < planes; p++) bad = bad || !tv[p]->ptr;
   if (bad) {
-    a.hot[idx] = CmdHot{};
+    wr_yuv_reject(a, idx);
     atomicAdd(&a.info->unsupported, 1);
     atomicAdd(a.err_counter, 1);
     return;
@@ -455,10 +573,11 @@ WRD void wr_setup_composite_yuv_one(const SetupArgs& a, int idx) {
       k->g[4 * p + 3] = (uvr[3] - 0.5f) / th;
     }
     wr_yuv_color_matrix(color_space, format, bit_depth, &k->g[12], &k->g[15]);
-    YuvFixed m = wr_yuv_fixed_from(&k->g[12], &k->g[15], 0);
+    YuvFixed m = wr_yuv_fixed_from(&k->g[12], &k->g[15], rescale);
     int* mi = (int*)(k->g + 24);
     mi[0] = m.bu; mi[1] = m.rv; mi[2] = m.gu; mi[3] = m.gv;
     mi[4] = m.y_coeff; mi[5] = m.y_bias; mi[6] = m.uv_bias; mi[7] = m.br_y_mask;
+    mi[9] = (16 - rescale - 1) - 8;  // rescaleBits (swgl_ext.h:1087-1088)
     k->i[0] = format;
     k->i[1] = planes;
     k->i[2] = -1;
@@ -506,12 +625,13 @@ WRD void wr_setup_brush_yuv_image_one(const SetupArgs& a, int idx) {
   const FrameTablesDev& T = a.tabs;
   float4 data = wr_fetch(T.gpu_cache, T.n_gpu_cache, vs.ph.specific_prim_address);
   int bit_depth = (int)data.x, color_space = (int)data.y, format = (int)data.z;
-  int planes = format == 3 ? 3 : (format == 0 ? 2 : (format == 4 ? 1 : 0));
+  int planes = wr_yuv_planes(format);
   const TexView* tv[3] = {&a.color0, &a.color1, &a.color2};
-  bool bad = bit_depth != 8 || planes == 0;
+  const int rescale = wr_yuv_rescale(format, bit_depth, tv);
+  bool bad = rescale < 0 || planes == 0;
   for (int p = 0; p < planes; p++) bad = bad || !tv[p]->ptr;
   if (bad) {
-    a.hot[idx] = CmdHot{};
+    wr_yuv_reject(a, idx);
     wr_finish_setup(a, 1);
     return;
   }
@@ -541,10 +661,11 @@ WRD void wr_setup_brush_yuv_image_one(const SetupArgs& a, int idx) {
       k->g[4 * p + 3] = (uvr[p].w - 0.5f) / th;
     }
     wr_yuv_color_matrix(color_space, format, bit_depth, &k->g[12], &k->g[15]);
-    YuvFixed m = wr_yuv_fixed_from(&k->g[12], &k->g[15], 0);
+    YuvFixed m = wr_yuv_fixed_from(&k->g[12], &k->g[15], rescale);
     int* mi = (int*)(k->g + 24);
     mi[0] = m.bu; mi[1] = m.rv; mi[2] = m.gu; mi[3] = m.gv;
     mi[4] = m.y_coeff; mi[5] = m.y_bias; mi[6] = m.uv_bias; mi[7] = m.br_y_mask;
+    mi[9] = (16 - rescale - 1) - 8;  // rescaleBits (swgl_ext.h:1087-1088)
     k->i[0] = format;
     k->i[1] = planes;
     k->i[2] = -1;
@@ -560,6 +681,7 @@ template <> struct WrRun<CompositeYuvShader> {  // brush_yuv_image draws under d
   enum { n = 6 };
   WRD_MEMBER int drawn(const CompositeYuvShader::Row& r) { return r.body_len; }
 };
+template <> struct WrRun<CompositeYuv16Shader> : WrRun<CompositeYuvShader> {};
 
 #ifndef WRCU_HOSTEMU
 // Strip mode: with the chain table the Row holds nothing that depends on the tile (the u sums come from the
@@ -568,6 +690,7 @@ template <> struct WrRowReuse<CompositeYuvShader> {
   enum { v = 1 };
   WRD_MEMBER bool ok(const CompositeYuvShader::Row& r) { return r.chain != nullptr; }
 };
+template <> struct WrRowReuse<CompositeYuv16Shader> : WrRowReuse<CompositeYuvShader> {};
 #endif
 
 #ifndef WRCU_HOSTEMU

@@ -42,7 +42,7 @@ typedef uint64_t GLuint64;
 enum {
   GL_NO_ERROR = 0, GL_INVALID_ENUM = 0x0500, GL_INVALID_VALUE = 0x0501, GL_INVALID_OPERATION = 0x0502,
   GL_OUT_OF_MEMORY = 0x0505,
-  GL_RGBA32F = 0x8814, GL_RGBA8 = 0x8058, GL_R8 = 0x8229, GL_RG8 = 0x822B, GL_RG = 0x8227, GL_RGBA32I = 0x8D82, GL_DEPTH_COMPONENT24 = 0x81A6,
+  GL_RGBA32F = 0x8814, GL_RGBA8 = 0x8058, GL_R8 = 0x8229, GL_RG8 = 0x822B, GL_R16 = 0x822A, GL_RG16 = 0x822C, GL_RG = 0x8227, GL_RGBA32I = 0x8D82, GL_DEPTH_COMPONENT24 = 0x81A6,
   GL_DEPTH_COMPONENT16 = 0x81A5, GL_DEPTH_COMPONENT32 = 0x81A7, GL_BGRA8 = 0x93A1,
   GL_BYTE = 0x1400, GL_UNSIGNED_BYTE = 0x1401, GL_SHORT = 0x1402, GL_UNSIGNED_SHORT = 0x1403, GL_INT = 0x1404, GL_FLOAT = 0x1406,
   GL_RED = 0x1903, GL_RGBA = 0x1908, GL_RGBA_INTEGER = 0x8D99, GL_BGRA = 0x80E1,
@@ -168,6 +168,8 @@ int wr_fmt(GLenum ifmt) {
     case GL_RGBA8: case GL_BGRA8: return WRCU_FMT_RGBA8;
     case GL_R8: return WRCU_FMT_R8;
     case GL_RG8: return WRCU_FMT_RG8;
+    case GL_R16: return WRCU_FMT_R16;
+    case GL_RG16: return WRCU_FMT_RG16;
     case GL_DEPTH_COMPONENT24: case GL_DEPTH_COMPONENT16: case GL_DEPTH_COMPONENT32: return WRCU_FMT_DEPTH24;
     default: return 0;
   }
@@ -176,7 +178,8 @@ int bytes_per_pixel(GLenum ifmt) {
   switch (ifmt) {
     case GL_RGBA8: case GL_BGRA8: return 4;
     case GL_R8: return 1;
-    case GL_RG8: return 2;
+    case GL_RG8: case GL_R16: return 2;
+    case GL_RG16: return 4;
     case GL_RGBA32F: case GL_RGBA32I: return 16;
     default: return 4;
   }

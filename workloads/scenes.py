@@ -1835,6 +1835,147 @@ def video_frame(width=3840, height=2160, vw=1920, vh=1080, fmt="nv12", color_spa
     return Frame(FrameTables().arrays(), textures, [[Target("fb", ops=ops)]])
 
 
+HDR_YUV_FORMATS = ("planar", "nv12", "p010")
+
+
+def hdr_yuv_planes(w, h, seed, fmt, depth):
+    """Seeded 10-, 12- or 16-bit video frame as 16-bit little-endian planes (uint8 rows): full-resolution luma,
+    4:2:0 chroma.  "planar": three R16 planes; "nv12": R16 + RG16 (CbCr interleaved); both LSB-aligned (codes
+    0 .. 2^depth - 1).  "p010": R16 + RG16 MSB-aligned (code << (16 - depth)), as P010 decoders write it."""
+    rng = np.random.RandomState(seed)
+    ph = rng.uniform(0, 6.28, 6)
+    top = (1 << depth) - 1
+
+    def plane(pw, ph_, k):
+        y2, x2 = np.mgrid[0:ph_, 0:pw].astype(np.float64)
+        v = 0.5 + 0.5 * np.sin(x2 / (11.0 + 7 * k) + ph[k]) * np.cos(y2 / (13.0 + 5 * k) + ph[3 + k])
+        v += rng.uniform(-0.06, 0.06, (ph_, pw))
+        # the full code range, so out-of-range samples exercise the saturating adds
+        return np.rint(np.clip(v, 0, 1) * top).astype(np.uint16)
+    cw, ch = (w + 1) // 2, (h + 1) // 2
+    y, u, v = plane(w, h, 0), plane(cw, ch, 1), plane(cw, ch, 2)
+    if fmt == "p010":
+        y, u, v = (p << (16 - depth) for p in (y, u, v))
+    rows = lambda p: p.view(np.uint8).reshape(p.shape[0], -1)  # noqa: E731
+    if fmt == "planar":
+        return [rows(y), rows(u), rows(v)]
+    return [rows(y), rows(np.ascontiguousarray(np.stack([u, v], axis=2)))]
+
+
+def _hdr_yuv_textures(fmt, vw, vh, seed, depth, filt):
+    """(plane names, YuvFormat, {name: TextureDesc}) of an hdr_yuv_planes frame"""
+    from webrender_b200.gpu_types import YUV_FORMAT_PLANAR, YUV_FORMAT_NV12, YUV_FORMAT_P010
+    planes = hdr_yuv_planes(vw, vh, seed, fmt, depth)
+    if fmt == "planar":
+        names, yuv_format, fmts = ("vy", "vu", "vv"), YUV_FORMAT_PLANAR, (abi.FMT_R16,) * 3
+    else:
+        names, yuv_format = ("vy", "vuv", ""), YUV_FORMAT_P010 if fmt == "p010" else YUV_FORMAT_NV12
+        fmts = (abi.FMT_R16, abi.FMT_RG16)
+    textures = {nm: TextureDesc(f, pl.shape[1] // abi.FMT_BPP[f], pl.shape[0], data=pl, filter=filt)
+                for nm, f, pl in zip(names, fmts, planes)}
+    return names, yuv_format, textures
+
+
+def hdr_yuv_composite_frame(fmt="p010", depth=10, color_space=2, seed=1, width=512, height=320, linear=True,
+                            opaque=True, fractional=False, right_edge=False):
+    """yuv_composite_frame's surfaces (1:1, whole frame scaled, sub-rects; flips and clips) from a 10-, 12- or
+    16-bit frame: PLANAR (three R16 planes), NV12 or P010 (R16 + RG16).  right_edge: every uv rect ends at the
+    planes' last texel column, where the 16-bit fetches weight the last texel by 127/128."""
+    from webrender_b200.gpu_types import composite_yuv_instance
+    rng = np.random.RandomState(seed * 37 + color_space + 100 * depth)
+    vw, vh = 192, 128
+    names, yuv_format, textures = _hdr_yuv_textures(fmt, vw, vh, seed + 5, depth, abi.LINEAR if linear else abi.NEAREST)
+    textures["fb"] = TextureDesc(abi.FMT_RGBA8, width, height)
+    insts = []
+    for i in range(6):
+        r = _rand_rect(rng, width, height, 40, 260, integer=not fractional)
+        ux, uy = float(2 * rng.randint(0, 30)), float(2 * rng.randint(0, 20))
+        if i == 0:      # 1:1
+            uw, uh = min(r[2] - r[0], vw - ux), min(r[3] - r[1], vh - uy)
+            uw, uh = float(int(uw) & ~1), float(int(uh) & ~1)
+            r = (r[0], r[1], r[0] + uw, r[1] + uh)
+        elif i == 1:    # the whole frame, scaled
+            ux, uy, uw, uh = 0.0, 0.0, float(vw), float(vh)
+        else:
+            uw, uh = float(2 * rng.randint(10, 60)), float(2 * rng.randint(8, 40))
+        if right_edge:
+            ux = float(vw) - uw
+        clip = r if i == 1 else (r[0] + 3.0, r[1] + 2.0, r[2] - 5.0, r[3] - 1.0)
+        ry = (ux, uy, ux + uw, uy + uh)
+        rc = tuple(v * 0.5 for v in ry)
+        insts.append(composite_yuv_instance(r, clip, color_space, yuv_format, depth, (ry, rc, rc), flip=(i == 3, i == 4)))
+    ops = [Clear(color=(0.1, 0.2, 0.3, 1.0)),
+           Batch(abi.KIND_COMPOSITE, np.stack(insts), blend=abi.BLEND_NONE if opaque else abi.BLEND_PREMULTIPLIED_ALPHA,
+                 features=abi.FEAT_TEXTURE_2D | abi.FEAT_YUV, color=names)]
+    return Frame(FrameTables().arrays(), textures, [[Target("fb", ops=ops)]])
+
+
+def hdr_yuv_image_frame(fmt="p010", depth=10, color_space=2, seed=1, width=512, height=320, linear=True,
+                        alpha_pass=True, fractional=False, with_masks=True, rotate=None):
+    """yuv_image_frame's Brush(YuvImage) primitives (opaque or alpha pass; AA edges, clip masks, a rotated node)
+    drawing a 10-, 12- or 16-bit frame: prim data [channel_bit_depth, colour space, format, 0]."""
+    from webrender_b200.gpu_types import brush_instance, CLIP_TASK_EMPTY
+    rng = np.random.RandomState(seed * 41 + color_space + 100 * depth)
+    t = FrameTables()
+    pic = t.add_render_task((0.0, 0.0, float(width), float(height)), 1.0, (0.0, 0.0))
+    vw, vh = 192, 128
+    names, yuv_format, textures = _hdr_yuv_textures(fmt, vw, vh, seed + 9, depth, abi.LINEAR if linear else abi.NEAREST)
+    textures["target"] = TextureDesc(abi.FMT_RGBA8, width, height)
+    xf = 0
+    if rotate is not None:
+        xf = t.add_transform(rotation_matrix(rotate, width / 2.0, height / 2.0, 1.0, 0.9), axis_aligned=False)
+    if with_masks and alpha_pass:
+        mask = rng.randint(0, 256, size=(256, 256)).astype(np.uint8)
+        mask[rng.randint(0, 256, 40)[:, None], :] = 255
+        mask[:, rng.randint(0, 256, 40)] = 0
+        textures["mask"] = TextureDesc(abi.FMT_R8, 256, 256, data=mask, filter=abi.NEAREST)
+    inst = []
+    for i in range(7):
+        r = _rand_rect(rng, width, height, 40, 240, integer=not fractional)
+        ux, uy = float(2 * rng.randint(0, 30)), float(2 * rng.randint(0, 20))
+        if i == 0:
+            uw, uh = float(int(min(r[2] - r[0], vw - ux)) & ~1), float(int(min(r[3] - r[1], vh - uy)) & ~1)
+            r = (r[0], r[1], r[0] + uw, r[1] + uh)
+        else:
+            uw, uh = float(2 * rng.randint(10, 60)), float(2 * rng.randint(8, 40))
+        ry = (ux, uy, ux + uw, uy + uh)
+        rc = tuple(v * 0.5 for v in ry)
+        srcs = [t.push_gpu_cache([rr, (0.0, 0.0, 0.0, 0.0)]) for rr in (ry, rc, rc)]
+        spec = t.push_gpu_cache([(float(depth), float(color_space), float(yuv_format), 0.0)])
+        clip = r if i % 3 else (r[0] + 4.0, r[1] + 3.0, r[2] - 6.0, r[3] - 2.0)
+        clip_task = CLIP_TASK_EMPTY
+        if with_masks and alpha_pass and i % 3 == 1:
+            w_, h_ = int(min(r[2] - r[0], 120)), int(min(r[3] - r[1], 100))
+            mx, my = int(rng.randint(0, 256 - w_)), int(rng.randint(0, 256 - h_))
+            clip_task = t.add_render_task((float(mx), float(my), float(mx + w_), float(my + h_)), 1.0,
+                                          (float(int(r[0])), float(int(r[1]))))
+        hdr = t.add_prim_header(r, clip, i + 1, spec, xf, pic, (srcs[0], srcs[1], srcs[2], 0))
+        edge = 0xF if (alpha_pass and (fractional or rotate is not None)) else 0
+        inst.append(brush_instance(hdr, clip_task, 0xFFFF, edge, 0, 0))
+    feats = abi.FEAT_TEXTURE_2D | abi.FEAT_YUV | (abi.FEAT_ALPHA_PASS if alpha_pass else 0)
+    ops = [Clear(color=(0.2, 0.3, 0.1, 1.0)),
+           Batch(abi.KIND_BRUSH_YUV_IMAGE, np.stack(inst),
+                 blend=abi.BLEND_PREMULTIPLIED_ALPHA if alpha_pass else abi.BLEND_NONE,
+                 features=feats, color=names, clip_mask="mask" if (with_masks and alpha_pass) else "")]
+    return Frame(t.arrays(), textures, [[Target("target", ops=ops)]])
+
+
+def hdr_video_frame(width=3840, height=2160, vw=1920, vh=1080, fmt="p010", depth=10, color_space=2, seed=1):
+    """video_frame with a 10-, 12- or 16-bit source: one vw x vh surface (P010 by default, Rec.709 narrow range)
+    scaled to the whole framebuffer by `composite` YUV."""
+    from webrender_b200.gpu_types import composite_yuv_instance
+    names, yuv_format, textures = _hdr_yuv_textures(fmt, vw, vh, seed, depth, abi.LINEAR)
+    textures["fb"] = TextureDesc(abi.FMT_RGBA8, width, height)
+    r = (0.0, 0.0, float(width), float(height))
+    ry = (0.0, 0.0, float(vw), float(vh))
+    rc = tuple(v * 0.5 for v in ry)
+    inst = composite_yuv_instance(r, r, color_space, yuv_format, depth, (ry, rc, rc))
+    ops = [Clear(color=(0.0, 0.0, 0.0, 1.0)),
+           Batch(abi.KIND_COMPOSITE, inst[None, :], blend=abi.BLEND_NONE,
+                 features=abi.FEAT_TEXTURE_2D | abi.FEAT_YUV, color=names)]
+    return Frame(FrameTables().arrays(), textures, [[Target("fb", ops=ops)]])
+
+
 def _picture_source(t, rng, aw, ah, w, h, one_to_one):
     """gpu-cache entry of an off-screen picture's uv rect the way
     RenderTaskCache/resolve_location publishes it: uv rect, user data, and the
